@@ -367,9 +367,14 @@ def run_b200(args, w):
     if ddp:
         ddp.average = mode != "sum"              # lambdaLoss(reduction="sum") gradients are summed across ranks
 
-    def step(x, y):
+    kept = {}
+
+    def step(x, y, keep=False):
         mask = y == PAD                                    # train_utils.py:19
-        loss = loss_fn(model(x, mask, None), y, **w["loss_args"])
+        scores = model(x, mask, None)
+        if keep:                                           # --dump-outputs: the scores of the last timed step
+            kept["scores"] = scores.detach().clone()
+        loss = loss_fn(scores, y, **w["loss_args"])
         loss.backward()
         scale = 1.0
         if ddp:
@@ -418,13 +423,16 @@ def run_b200(args, w):
     l0 = _lib.launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(args.steps):
-        loss = gstep.replay() if gstep else step(x_dev, y_dev)
+    for i in range(args.steps):
+        loss = gstep.replay() if gstep else step(x_dev, y_dev, keep=args.dump_outputs and i == args.steps - 1)
     e1.record()
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     launches = launches_per_replay * args.steps if gstep else _lib.launch_count() - l0
     final_loss = loss.item()
+    if args.dump_outputs and rank == 0:                    # before the steps below move the parameters on
+        kept.update(loss=loss.detach().reshape(1), parameters=model.flat_parameters)
+        kept = {k: v.float().cpu().numpy() for k, v in kept.items()}
 
     # ---- (2) end to end: every step's inputs come from pinned host memory (H2D inside the timed region, issued on
     #      a copy stream one step ahead, the way a training loop with a prefetching loader runs) and the loss is
@@ -556,9 +564,30 @@ def run_b200(args, w):
         }
     if world == 1 and not args.no_cpu_baseline:
         out["cpu_baseline"] = cpu_baseline_subprocess(args, w)
+    if args.dump_outputs:
+        out["dumped"] = dump_outputs(args.dump_outputs, kept)
     print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_MAX_ELEMENTS = 4 << 20     # per array: 16 MB of float32, so that a dump stays within 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Write each array as <path>/<name>.npy (float32).  An array longer than DUMP_MAX_ELEMENTS is replaced by the
+    same fixed, seeded sample of its flattened entries in every run, so that two builds compare entry for entry."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    written = {}
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.size > DUMP_MAX_ELEMENTS:
+            pick = np.sort(np.random.RandomState(0).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))
+            a = a.reshape(-1)[pick]
+        np.save(os.path.join(path, name + ".npy"), a)
+        written[name] = list(a.shape)
+    return written
 
 
 def measured_traffic(args, batch, kernel):
@@ -598,8 +627,14 @@ def main():
     ap.add_argument("--cuda-graph", action="store_true",
                     help="replay the training step as one CUDA graph (allrank_b200.graph.GraphedTrainStep; one GPU, "
                          "flat optimiser): for small batches, where the host's launch path sets the pace")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the last one computed -- the scores, the loss and the "
+                         "updated parameters (no scores with --cuda-graph) -- as DIR/<name>.npy (float32); inputs are "
+                         "seeded, so runs compare")
     ap.add_argument("--allow-short-warmup", action="store_true", help="(internal: the bounded CPU leg)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and not args.allow_short_warmup:
         args.warmup = 3
     w = WORKLOADS[args.workload]

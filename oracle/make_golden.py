@@ -217,8 +217,44 @@ def gen_scorer():
         (model(x, mask, idx) * (w * (~mask).float())).sum().backward()
         for k_, p in model.named_parameters():
             blob["gv:" + k_] = p.grad.numpy().copy()
+        if sum(p.numel() for p in model.parameters()) > COMPACT_ABOVE_PARAMS:
+            blob = compact_scorer_blob(blob, init_seed=7, perturb_seed=11, slates=(31, 0.6 * S, 0.3 * S))
         np.savez_compressed(os.path.join(OUT, f"scorer_{name}.npz"), **blob)
         print("scorer", name, "scores", tuple(scores.shape))
+
+
+COMPACT_ABOVE_PARAMS = 100_000
+GRAD_KEEP = 1024
+
+
+def compact_scorer_blob(blob, init_seed, perturb_seed, slates):
+    """Keep a golden scorer file small.  The parameters and the features are not stored: tests/conftest.py rebuilds
+    the parameters with allrank_b200's make_model under torch.manual_seed(init_seed) -- the reference's seeded
+    initialisation, pinned by tests/test_host_model.py -- and the 1-D shift drawn from perturb_seed, and the features
+    with make_slates(seed, mean_len, std_len) = `slates` (both checked here).  A gradient of more than GRAD_KEEP
+    entries is kept at GRAD_KEEP fixed, seeded flat positions, stored as gi:<name>."""
+    from allrank_b200.model import make_model
+    F, d, N, h, dff = [int(v) for v in blob["meta"][:5]]
+    act = str(blob["act"])
+    torch.manual_seed(init_seed)
+    model = make_model(fc_model={"sizes": [d], "input_norm": False, "activation": None, "dropout": 0.0},
+                       transformer={"N": N, "d_ff": dff, "h": h, "positional_encoding": None, "dropout": 0.0},
+                       post_model={"d_output": 1, "output_activation": None if act == "None" else act}, n_features=F)
+    perturb_vectors(model, perturb_seed)
+    for k_, v in model.state_dict().items():
+        assert np.array_equal(v.numpy(), blob.pop("p:" + k_)), k_
+    B, S = [int(v) for v in blob["meta"][5:7]]
+    x, y, _ = make_slates(B, S, n_features=F, seed=slates[0], mean_len=slates[1], std_len=slates[2])
+    assert np.array_equal(x.numpy(), blob.pop("x")) and np.array_equal(y.numpy(), blob["y"])
+    out = dict(blob, init_seed=np.array(init_seed), perturb_seed=np.array(perturb_seed), slates=np.array(slates))
+    for k_, v in blob.items():
+        if k_.startswith("g:") and v.size > GRAD_KEEP:
+            name = k_[2:]
+            idx = np.sort(np.random.RandomState(0).choice(v.size, GRAD_KEEP, replace=False)).astype(np.int32)
+            out["gi:" + name] = idx
+            out["g:" + name] = v.reshape(-1)[idx]
+            out["gv:" + name] = blob["gv:" + name].reshape(-1)[idx]
+    return out
 
 
 def gen_scorer_pe():
@@ -467,9 +503,69 @@ def gen_init():
     print("init:", len(blob), "tensors")
 
 
+def gen_l3():
+    """The reference's own run() (oracle/run_reference_main.py, on the CPU) for the two training configs of
+    tests/test_gpu_l3_training.py, checked against oracle/train_ref.py driving the reference's components."""
+    import json
+    import subprocess
+    import tempfile
+    from allrank.models.model import make_model
+    from allrank.training.train_utils import compute_metrics
+    from oracle import train_ref
+
+    def ref_make_model(n_features, fc_model, transformer, post_model):
+        return make_model(n_features=n_features, fc_model=fc_model, post_model=post_model,
+                          transformer=TransformerConfig(**transformer) if transformer else None)
+
+    out = {}
+    for name in ("baseline_cfg1", "transformer_cfg"):
+        config = os.path.join(ROOT, "tests", "configs", name + ".json")
+        with tempfile.TemporaryDirectory() as tmp:
+            r = subprocess.run([sys.executable, os.path.join(HERE, "run_reference_main.py"), "--workdir", tmp,
+                                "--config", config, "--run-id", "cpu"], stdout=subprocess.PIPE, text=True, check=True)
+            res = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("RESULT ")][-1][len("RESULT "):])
+            res.pop("native_so_loaded")
+            with open(config) as fh:
+                port = train_ref.run(json.load(fh), os.path.join(tmp, "dummy_data"), torch.device("cpu"),
+                                     ref_make_model, ref_losses, compute_metrics)
+        flat = {"epochs": port["epochs"], "num_params": port["num_params"]}
+        for role in ("train", "val"):
+            flat.update({f"{role}_metrics/{k}": v for k, v in port[role + "_metrics"].items()})
+        assert flat == res, (name, flat, res)
+        out[name] = res
+    with open(os.path.join(OUT, "l3_reference.json"), "w") as fh:
+        json.dump(out, fh, indent=1, sort_keys=True)
+    print("l3:", out)
+
+
+def gen_reference_api():
+    """Parameter names of the reference callables allrank_b200.integration rebinds, and the padding constants."""
+    import inspect
+    import json
+    import allrank.data.dataset_loading as ref_dl
+    from allrank_b200 import integration
+    names = {"allrank.models.losses": integration.LOSS_NAMES, "allrank.models.metrics": integration.METRIC_NAMES,
+             "allrank.models.model": ("make_model",),
+             "allrank.training.train_utils": ("metric_on_batch", "metric_on_epoch", "compute_metrics"),
+             "allrank.inference.inference_utils": ("rank_slates",),
+             "allrank.data.dataset_loading": ("load_libsvm_dataset", "load_libsvm_dataset_role", "load_libsvm_role",
+                                              "create_data_loaders"),
+             "allrank.main": ("make_model", "load_libsvm_dataset", "create_data_loaders", "CustomDataParallel")}
+    sig = {}
+    for mod, fns in names.items():
+        m = __import__(mod, fromlist=["_"])
+        sig[mod] = {n: None if inspect.isclass(getattr(m, n)) else list(inspect.signature(getattr(m, n)).parameters)
+                    for n in fns}
+    consts = {"PADDED_Y_VALUE": ref_dl.PADDED_Y_VALUE, "PADDED_INDEX_VALUE": ref_dl.PADDED_INDEX_VALUE}
+    with open(os.path.join(OUT, "reference_api.json"), "w") as fh:
+        json.dump({"signatures": sig, "dataset_loading_constants": consts}, fh, indent=1)
+    print("reference api:", sum(len(v) for v in sig.values()), "callables")
+
+
 if __name__ == "__main__":
     torch.set_num_threads(4)
     gens = {"losses": gen_losses, "listmle": gen_listmle, "bce": gen_bce, "ordinal": gen_ordinal, "metrics": gen_metrics,
-            "scorer": gen_scorer, "scorer_pe": gen_scorer_pe, "scorer_multi": gen_scorer_multi, "scorer_shipped": gen_scorer_shipped, "neural_sort": gen_neural_sort, "slates": gen_slates, "init": gen_init}
+            "scorer": gen_scorer, "scorer_pe": gen_scorer_pe, "scorer_multi": gen_scorer_multi, "scorer_shipped": gen_scorer_shipped, "neural_sort": gen_neural_sort, "slates": gen_slates, "init": gen_init,
+            "l3": gen_l3, "reference_api": gen_reference_api}
     for name in (sys.argv[1:] or list(gens)):      # optionally: only the named generators
         gens[name]()
